@@ -4,6 +4,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this framework (CUDA path), DDPG (BASELINE configs[1])
   python bench.py --algo td3 ...                           # the same line for TD3 (BASELINE configs[2])
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's losses and weights
   python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host cores
                                                            # (numpy port in oracle/; /root/reference is Python
                                                            # and does not exist on the GPU box)
@@ -347,6 +348,16 @@ class Bench:
         return {"ms": rep_ms, "kernels": int(kernels), "loss": loss, "wall_s": wall}
 
 
+def timed_outputs(agent, loss):
+    """What a caller of the timed path holds after its last step: the dict update() returned and every net's
+    weights (updated in place), as host float64 / float32 arrays keyed by output file name."""
+    out = {"loss.%s" % k: np.asarray(v, dtype=np.float64) for k, v in loss.items()}
+    for net, module in sorted(agent.nets.items()):
+        for k, p in module.state_dict().items():
+            out["%s.%s" % (net, k)] = p.detach().float().cpu().numpy()
+    return out
+
+
 def summarize(rep_ms, steps, world):
     """steps/s per repeat -> median (whole job: x world 4096-row minibatches), min, max."""
     v = sorted(steps / (m / 1e3) * world for m in rep_ms)
@@ -456,6 +467,7 @@ def run_native(args):
         sampler.start()
     r_dev = main.run(False, steps, warmup, repeats)
     clocks = sampler.stop() if rank == 0 else {}
+    dump = timed_outputs(main.agent, r_dev["loss"]) if (args.dump_outputs and rank == 0) else None
     r_e2e = main.run(True, steps, 3, repeats)
     r_warm = main.run(False, steps, 3, 1, flush_l2=False)
     value, spread = summarize(r_dev["ms"], steps, world)
@@ -681,6 +693,10 @@ def run_native(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if line is not None:
         print(json.dumps(line))
 
@@ -802,10 +818,14 @@ def main():
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu_baseline legs (A/B runs)")
     ap.add_argument("--no-other-algo", action="store_true", help="skip the sub-object of the other algorithm")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (losses) and left in the nets (weights, ~7 MB for "
+                         "DDPG, ~10 MB for TD3) as DIR/<name>.npy; the inputs are seeded, so runs with the same "
+                         "arguments can be compared output for output")
     args = ap.parse_args()
     if args.impl == "reference":
-        if args.steps > 40:          # bounded: the CPU port does ~3-10 steps/s
-            args.steps = 40
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl native")
         args.warmup = min(args.warmup, 3)
         run_reference(args)
     else:

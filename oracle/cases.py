@@ -32,6 +32,34 @@ CASES = {
 FULL_SPEC = dict(seeds={"ddpg": 11, "td3": 12}, n_items=26744, dim=128, frame=10, hidden=256, n_rows=4096,
                  steps=3, actor_init_w=6e-1, critic_init_w=54e-2)
 
+
+def _unscreened(seed, **kw):
+    spec = dict(CASES["tiny"], steps=12)
+    spec["seeds"] = {"ddpg": seed, "td3": seed + 1}
+    spec.update(kw)
+    return spec
+
+
+# Seeds that were NOT screened by oracle/find_seeds.py, at shapes other than CASES': the oracle is compared on them
+# with vectors recorded from the reference (tests/golden/vs_reference.npz, oracle/make_golden.py).
+UNSCREENED_CASES = {
+    "tiny-a": _unscreened(1001),
+    "narrow": _unscreened(1002, n_rows=17, dim=8, frame=3, hidden=16, n_items=40),
+    "wide": _unscreened(1003, n_rows=40, hidden=64),
+}
+UNSCREENED_SAMPLES = 32         # leading entries of each net_digest sample kept for these cases (file size)
+
+
+def random_gather_users():
+    """table, ragged users and frame size of the gather comparison in tests/golden/vs_reference.npz."""
+    rng = np.random.default_rng(31)
+    frame = 7
+    table = rng.standard_normal((90, 12), dtype=np.float32)
+    users = [{"items": rng.integers(0, 90, size=n, dtype=np.int64), "rates": rng.standard_normal(n) * 2,
+              "sizes": n, "users": 5 + i} for i, n in enumerate((8, 30, 9, 8, 21))]
+    return table, users, frame
+
+
 DDPG_PARAMS = dict(gamma=0.99, min_value=-10, max_value=10, policy_step=10, soft_tau=0.001)  # algo.py:103-109
 TD3_PARAMS = dict(gamma=0.99, noise_std=0.5, noise_clip=3, soft_tau=0.001, policy_update=10)  # algo.py:164-174
 

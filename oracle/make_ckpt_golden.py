@@ -9,8 +9,8 @@ available offline, so the fixture is the same artefact made here: state_dicts of
 (constructed by the reference, reduced dims to keep the fixture small), saved with torch.save exactly as the
 reference does, plus eval-mode inputs and the REFERENCE's forward outputs on them.
 tests/test_checkpoint_compat.py loads the file into recnn_b200.nn.Actor / Critic (CUDA forward must reproduce the
-stored outputs) and checks that a state_dict saved by recnn_b200 loads back into the reference classes (same keys,
-shapes, dtypes, contiguous tensors).
+stored outputs) and checks that a state_dict saved by recnn_b200 has the layout of the reference classes' own
+(same keys in the same order, shapes, dtypes), so that they load it with strict=True.
 """
 from __future__ import annotations
 

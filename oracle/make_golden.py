@@ -30,6 +30,9 @@ are produced here by differential execution of its own functions):
   every parameter of every net after steps {1, 2, 11, 12}, critic .grad after
   step index 1 (a non-policy step: pure value-loss gradient) and actor .grad
   after step index 0 (post "clip": sign-flipped, L1-normalised).
+* vs_reference.npz -- the same update cases on the unscreened seeds and shapes of
+                 C.UNSCREENED_CASES, and the gather on C.random_gather_users(),
+                 reduced to what tests/test_oracle_vs_reference.py compares.
 """
 from __future__ import annotations
 
@@ -194,6 +197,38 @@ def run_update_case(recnn, case, algo, opt_kind):
     return out
 
 
+def run_vs_reference_cases(recnn):
+    """vs_reference.npz: the update cases of C.UNSCREENED_CASES (keys '<case>.<algo>.<opt>.*') and the gather on
+    C.random_gather_users() ('gather.*'), both run by the reference.  Only what tests/test_oracle_vs_reference.py
+    compares is kept: losses, input checksums, the gate margin, TD3's noise draws ('<case>.noise' [steps, rows,
+    dim], the same for both optimizers) and the first C.UNSCREENED_SAMPLES entries of each weight sample (and of
+    DDPG's gradient samples), concatenated in the order of 'sample_keys' with lengths 'sample_sizes'.  A case with
+    an ambiguous ReLU gate, which the test skips, keeps its gate margin only."""
+    out = {}
+    for name, spec in C.UNSCREENED_CASES.items():
+        for algo in ("ddpg", "td3"):
+            for opt_kind in ("adam", "sgd"):
+                got = run_update_case(recnn, spec, algo, opt_kind)
+                pre = "%s.%s.%s." % (name, algo, opt_kind)
+                out[pre + "gate_margin"] = got["gate_margin"]
+                if float(got["gate_margin"]) <= C.GATE_GUARD:
+                    continue
+                for k in ["input_checksums"] + [k for k in got if k.startswith("loss.")]:
+                    out[pre + k] = got[k]
+                if algo == "td3":
+                    out[name + ".noise"] = np.stack([got["noise.%d" % s] for s in range(spec["steps"])])
+                keys = sorted(k for k in got if k.endswith(".sample") and (algo == "ddpg" or not k.startswith("grad_")))
+                samples = [got[k][:C.UNSCREENED_SAMPLES] for k in keys]
+                out[pre + "sample_keys"] = np.asarray(keys)
+                out[pre + "sample_sizes"] = np.asarray([s.size for s in samples], dtype=np.int64)
+                out[pre + "samples"] = np.concatenate(samples)
+    table, users, frame = C.random_gather_users()
+    ref = recnn.data.utils.prepare_batch_static_size(copy.deepcopy(users), torch.from_numpy(table), frame_size=frame)
+    for k in ("state", "next_state", "action", "reward", "done"):
+        out["gather." + k] = ref[k].numpy()
+    return out
+
+
 def run_gather_case(recnn):
     rng = np.random.default_rng(2024)
     frame = 10
@@ -315,6 +350,9 @@ def main():
     if not only or "collate" in only:
         np.savez_compressed(os.path.join(GOLDEN_DIR, "collate.npz"), **run_collate_case(recnn))
         print("wrote collate.npz")
+    if not only or "vs_reference" in only:
+        np.savez_compressed(os.path.join(GOLDEN_DIR, "vs_reference.npz"), **run_vs_reference_cases(recnn))
+        print("wrote vs_reference.npz")
     if only and "gather" not in only and "update" not in only:
         return
     if not only or "gather" in only:

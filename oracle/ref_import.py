@@ -1,8 +1,8 @@
-"""Import the UNMODIFIED reference (awarebayes/RecNN) from /root/reference.
+"""Import the UNMODIFIED reference (awarebayes/RecNN) from a local checkout.
 
-TEST INFRASTRUCTURE.  Only usable in the build container (the GPU box has no
-/root/reference); used by ``oracle/make_golden.py`` and by the optional
-``tests/test_oracle_vs_reference.py`` (skipped when the tree is absent).
+TEST INFRASTRUCTURE.  Only usable where a checkout of the reference exists
+(``RECNN_REFERENCE_ROOT``); used by the generators of ``tests/golden/``
+(``oracle/make_*golden.py``).  No test imports it.
 
 Two modules the reference imports at package-import time are not installed
 here and are off the hot path (SURVEY.md 8c): ``matplotlib`` (pulled in by

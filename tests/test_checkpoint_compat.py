@@ -42,26 +42,26 @@ def test_saved_state_dict_round_trips_through_torch_save(tmp_path):
         assert torch.equal(back[k], v) and back[k].is_contiguous() and tuple(back[k].shape) == tuple(v.shape)
 
 
-def test_saved_state_dict_loads_into_the_reference_classes():
-    from oracle.ref_import import reference_available, import_reference
-    if not reference_available():
-        pytest.skip("reference tree not present (GPU box)")
-    import sys
-    before = set(sys.modules)
-    try:
-        recnn = import_reference()
-        ck = _load()
-        S, A, H = ck["dims"]
-        ours = recnn_b200.nn.Actor(S, A, H)
-        ours.load_state_dict(ck["actor"])
-        theirs = recnn.nn.models.Actor(S, A, H).eval()
-        theirs.load_state_dict(ours.state_dict(), strict=True)
-        with torch.no_grad():
-            assert torch.equal(theirs(ck["state"]), ck["out"]["actor"])
-    finally:          # leave no 'recnn' behind: tests/test_host.py registers recnn_b200 under that name
-        for name in set(sys.modules) - before:
-            if name == "recnn" or name.startswith("recnn."):
-                del sys.modules[name]
+def test_saved_state_dict_loads_into_the_reference_classes(tmp_path):
+    """The fixture's state_dicts were written by the reference's own Actor / Critic, so they record what its
+    load_state_dict(strict=True) accepts: these keys in this order, these shapes and dtypes.  A file saved by
+    recnn_b200 must match that layout, and after loading the fixture it must carry the very weights on which the
+    reference computed ck["out"]."""
+    ck = _load()
+    S, A, H = ck["dims"]
+    for kind, cls in (("actor", recnn_b200.nn.Actor), ("critic", recnn_b200.nn.Critic)):
+        ref = ck[kind]
+        for loaded in (False, True):
+            ours = cls(S, A, H)
+            if loaded:
+                ours.load_state_dict(ref)
+            path = tmp_path / ("%s_%d.model" % (kind, loaded))
+            torch.save(ours.state_dict(), path)
+            back = torch.load(path, map_location="cpu", weights_only=True)
+            assert list(back.keys()) == list(ref.keys()), kind
+            for k, v in ref.items():
+                assert tuple(back[k].shape) == tuple(v.shape) and back[k].dtype == v.dtype, (kind, k)
+                assert not loaded or torch.equal(back[k], v), (kind, k)
 
 
 @pytest.mark.gpu

@@ -23,11 +23,11 @@ def test_library_exports_every_declared_symbol():
     header = open(os.path.join(ROOT, "include", "recnn_b200.h")).read()
     declared = set(re.findall(r"RECNN_API\s+[\w\s\*]+?\b(recnn_\w+)\s*\(", header))
     assert len(declared) >= 15
+    L = _lib.lib()                       # builds the library if missing; also verifies struct size / offsets
     handle = ctypes.CDLL(_lib.lib_path())
     for name in declared:
         assert hasattr(handle, name), name
     assert declared == set(_lib.SIGNATURES), declared ^ set(_lib.SIGNATURES)
-    L = _lib.lib()                       # also verifies struct size / offsets
     assert L.recnn_b200_abi_version() == 3
     assert L.recnn_sizeof_step_args() == ctypes.sizeof(_lib.StepArgs)
 
