@@ -356,6 +356,19 @@ RECNN_API int recnn_reinforce_policy_grad(const recnn_discrete_dims* d, const fl
                                           const float* state, const int64_t* action, const float* beta_log_prob,
                                           const float* returns, int64_t n_rows, int32_t method, int32_t top_k,
                                           float* out, float* scratch, void* stream);
+/* Item-streamed form of recnn_reinforce_policy_grad for vocabularies whose [n_rows, num_items] logits do not fit in
+ * memory (reinforce.py:10-65 with models.py:95-99 over a million items): the same arguments and outputs, plus
+ * item_chunk >= 1.  The logits are computed item_chunk items at a time (the last chunk may be narrower) twice -- once
+ * for each row's softmax statistics and the log-prob of its action, once more for d loss / d logits, consumed chunk by
+ * chunk by the weight and hidden-layer gradients -- so the scratch holds one [n_rows, item_chunk] chunk instead of all
+ * logits.  Deterministic for a given item_chunk; about 4/3 the logit FLOPs of the materialised entry. */
+RECNN_API int64_t recnn_reinforce_streamed_scratch_floats(const recnn_discrete_dims* d, int64_t n_rows,
+                                                          int32_t item_chunk);
+RECNN_API int recnn_reinforce_policy_grad_streamed(const recnn_discrete_dims* d, const float* params, float* grads,
+                                                   const float* state, const int64_t* action,
+                                                   const float* beta_log_prob, const float* returns, int64_t n_rows,
+                                                   int32_t method, int32_t top_k, int32_t item_chunk, float* out,
+                                                   float* scratch, void* stream);
 
 /* ---- data parallel: all-reduce over NVLink peer memory ------------------------------------------
  * BASELINE north_star: "partition the embedding gather + update across the 8 GPUs of one box with

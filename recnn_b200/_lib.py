@@ -116,6 +116,10 @@ SIGNATURES = {
     "recnn_reinforce_policy_grad": (C.c_int, [C.POINTER(DiscreteDims), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
                                               C.c_void_p, C.c_void_p]),
+    "recnn_reinforce_streamed_scratch_floats": (C.c_int64, [C.POINTER(DiscreteDims), C.c_int64, C.c_int32]),
+    "recnn_reinforce_policy_grad_streamed": (C.c_int, [C.POINTER(DiscreteDims), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
+                                                       C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "recnn_comm_create": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, C.POINTER(C.c_void_p)]),
     "recnn_comm_handle_bytes": (C.c_int32, []),
     "recnn_comm_local_handle": (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -41,7 +41,9 @@ enum EpiKind {
   EPI_LINEAR = 1,   // out = acc + bias[n] (+tanh) (+clamp(noise))       (models.py:70-72, td3.py:74-78)
   EPI_GATE = 2,     // out = acc * (h[m,n] > 0 ? gate_scale : 0)          (relu'/dropout backward)
   EPI_STORE = 3,    // out = acc
-  EPI_PARTIAL = 4   // split-K partial: part[z][m][n] = acc
+  EPI_PARTIAL = 4,  // split-K partial: part[z][m][n] = acc
+  EPI_DLOGITS = 5,  // out = g[m] ([col0 + n == a[m]] - exp(acc + bias[n] - M[m]) / S[m])   (REINFORCE d logits)
+  EPI_ACCUM = 6     // out += acc, then (h given) the EPI_GATE gate of the sum
 };
 
 struct Epilogue {
@@ -61,7 +63,20 @@ struct Epilogue {
   float noise_clip;
   float noise_std;       // perf mode: philox normal * std (noise == null && add_noise)
   int add_noise;
+  // EPI_DLOGITS: per-row softmax statistics of the full item range, the row's dL/dlp and drawn action; output column n
+  // is item col0 + n
+  const float* row_g;
+  const float* row_max;
+  const float* row_sum;
+  const long long* row_action;
+  long long col0;
 };
+
+// d loss / d logit of one item from its logit z (the same fp32 operations as the materialised path's
+// softmax_rows_kernel + reinforce_dlogits_kernel)
+__device__ __forceinline__ float dlogit(float g, float z, float M, float S, bool is_action) {
+  return g * ((is_action ? 1.f : 0.f) - expf(z - M) / S);
+}
 
 template <int EPI>
 __device__ __forceinline__ void epi_store(const Epilogue& e, int M, int N, int m, int n, float acc, int z) {
@@ -100,6 +115,11 @@ __device__ __forceinline__ void epi_store(const Epilogue& e, int M, int N, int m
     }
   } else if (EPI == EPI_GATE) {
     v = e.h[(long long)m * e.ldh + n] > 0.f ? v * e.gate_scale : 0.f;
+  } else if (EPI == EPI_DLOGITS) {
+    v = dlogit(e.row_g[m], v + e.bias[n], e.row_max[m], e.row_sum[m], e.col0 + n == e.row_action[m]);
+  } else if (EPI == EPI_ACCUM) {
+    v = e.out[(long long)m * e.ldo + n] + v;
+    if (e.h) v = e.h[(long long)m * e.ldh + n] > 0.f ? v * e.gate_scale : 0.f;
   }
   e.out[(long long)m * e.ldo + n] = v;
 }

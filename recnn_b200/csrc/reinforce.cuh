@@ -14,6 +14,9 @@
 //   * d loss / d logits has a closed form (softmax + log + the scalar weight of the row), so the backward starts from
 //     ONE in-place row kernel that turns the probabilities into d logits; the rest is the usual three GEMMs.
 //   * the normalised discounted returns (reinforce.py:44-52) are T scalars: host arithmetic in the caller.
+//   * past what the [R, num_items] logits can hold (1M items), recnn_reinforce_policy_grad_streamed recomputes them one
+//     item chunk at a time: a statistics pass (online softmax max / sum, the action's logit) and a backward pass whose
+//     GEMM epilogue writes d logits (EPI_DLOGITS) for the chunk's dW2 and its term of dh.
 //
 // Per saved row n with sampled action a, p = clamp(pi[a], eps, 1-eps), lp = log p, R = return of the row's step:
 //   basic   (reinforce.py:16-22)   L = -lp R                                 dL/dlp = -R
@@ -177,6 +180,32 @@ __global__ void categorical_log_prob_kernel(const float* __restrict__ probs, lon
   }
 }
 
+// Row r's term L of the policy loss and g = dL / d log pi[a], from the probability pa = pi[a] of its drawn action (the
+// closed forms at the top of this file).  Both the materialised and the item-streamed policy gradient call this.
+__device__ __forceinline__ void reinforce_row_terms(float pa, long long r, const float* __restrict__ beta_logp,
+                                                    const float* __restrict__ ret, int method, int K, float& L, float& g) {
+  const float p = fminf(fmaxf(pa, kProbEps), 1.f - kProbEps);
+  const bool inside = pa > kProbEps && pa < 1.f - kProbEps;       // the clamp has zero slope outside
+  const float lp = logf(p), R = ret[r];
+  if (method == RECNN_REINFORCE_BASIC) {
+    L = -lp * R;
+    g = -R;
+  } else {
+    const float c = p / expf(beta_logp[r]);
+    if (method == RECNN_REINFORCE_CORRECTED) {
+      L = c * -lp * R;
+      g = -R * c * (lp + 1.f);
+    } else {
+      const float q = 1.f - p, Kf = (float)K;
+      const float lam = Kf * powf(q, Kf - 1.f);
+      const float dlam = K > 1 ? -Kf * (Kf - 1.f) * powf(q, Kf - 2.f) * p : 0.f;      // d lam / d lp
+      L = lam * c * -lp * R;
+      g = -R * c * (dlam * lp + lam * (lp + 1.f));
+    }
+  }
+  if (!inside) g = 0.f;
+}
+
 // probabilities -> d loss / d logits, in place; row_loss[r] = this row's term of the policy loss.
 __global__ void __launch_bounds__(kRowThreads)
 reinforce_dlogits_kernel(float* __restrict__ z, long long ld, long long n, int items, const long long* __restrict__ action,
@@ -192,29 +221,7 @@ reinforce_dlogits_kernel(float* __restrict__ z, long long ld, long long n, int i
     }
     if (threadIdx.x == 0) {
       float g = 0.f, L = 0.f;
-      if (a >= 0) {
-        const float pa = row[a];
-        const float p = fminf(fmaxf(pa, kProbEps), 1.f - kProbEps);
-        const bool inside = pa > kProbEps && pa < 1.f - kProbEps;       // the clamp has zero slope outside
-        const float lp = logf(p), R = ret[r];
-        if (method == RECNN_REINFORCE_BASIC) {
-          L = -lp * R;
-          g = -R;
-        } else {
-          const float c = p / expf(beta_logp[r]);
-          if (method == RECNN_REINFORCE_CORRECTED) {
-            L = c * -lp * R;
-            g = -R * c * (lp + 1.f);
-          } else {
-            const float q = 1.f - p, Kf = (float)K;
-            const float lam = Kf * powf(q, Kf - 1.f);
-            const float dlam = K > 1 ? -Kf * (Kf - 1.f) * powf(q, Kf - 2.f) * p : 0.f;      // d lam / d lp
-            L = lam * c * -lp * R;
-            g = -R * c * (dlam * lp + lam * (lp + 1.f));
-          }
-        }
-        if (!inside) g = 0.f;
-      }
+      if (a >= 0) reinforce_row_terms(row[a], r, beta_logp, ret, method, K, L, g);
       s_g = g;
       row_loss[r] = L;
     }
@@ -223,6 +230,65 @@ reinforce_dlogits_kernel(float* __restrict__ z, long long ld, long long n, int i
     for (int j = threadIdx.x; j < items; j += blockDim.x) row[j] = g * ((j == a ? 1.f : 0.f) - row[j]);
     __syncthreads();
   }
+}
+
+// ---- item-streamed policy gradient: the logits of one item chunk at a time, per-row statistics in between
+// Statistics pass, one chunk: z [n, cw] holds the logits of items c0 .. c0+cw.  Merges the chunk into the row's running
+// max M and sum S of exp(z - M) (online softmax: M' = max(M, m_c), S' = S e^(M - M') + s_c e^(m_c - M')) and records the
+// logit of the row's drawn action when it lies in the chunk.  One CTA per row; the reduction order is fixed.
+__global__ void __launch_bounds__(kRowThreads)
+reinforce_chunk_stats_kernel(const float* __restrict__ z, long long n, int cw, long long c0, int first,
+                             const long long* __restrict__ action, float* __restrict__ row_max,
+                             float* __restrict__ row_sum, float* __restrict__ za) {
+  __shared__ float red[32];
+  for (long long r = blockIdx.x; r < n; r += gridDim.x) {
+    const float* row = z + r * cw;
+    float m = -INFINITY, s = 0.f;
+    for (int j = threadIdx.x; j < cw; j += blockDim.x) {      // as softmax_rows_kernel
+      const float x = row[j];
+      if (x > m) {
+        s = s * __expf(m - x) + 1.f;
+        m = x;
+      } else {
+        s += __expf(x - m);
+      }
+    }
+    const float mc = block_max(m, red);
+    s = (m == -INFINITY) ? 0.f : s * __expf(m - mc);
+    const float sc = block_sum(s, red);
+    if (threadIdx.x == 0) {
+      if (first) {
+        row_max[r] = mc;
+        row_sum[r] = sc;
+      } else {
+        const float M = row_max[r], M2 = fmaxf(M, mc);
+        row_sum[r] = row_sum[r] * __expf(M - M2) + sc * __expf(mc - M2);
+        row_max[r] = M2;
+      }
+      const long long a = action[r] - c0;
+      if (a >= 0 && a < cw) za[r] = row[a];
+    }
+    __syncthreads();
+  }
+}
+
+// After the statistics pass: pi[a] = exp(z_a - M) / S, the row's loss term and g = dL / d log pi[a].  One thread per row.
+__global__ void reinforce_streamed_terms_kernel(long long n, int items, const long long* __restrict__ action,
+                                                const float* __restrict__ row_max, const float* __restrict__ row_sum,
+                                                const float* __restrict__ za, const float* __restrict__ beta_logp,
+                                                const float* __restrict__ ret, int method, int K,
+                                                float* __restrict__ row_loss, float* __restrict__ row_g, int* oob) {
+  const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const long long a = action[r];
+  float L = 0.f, g = 0.f;
+  if (a < 0 || a >= items) {            // an id outside the policy's output layer: flagged, contributes nothing
+    if (oob) *oob = 1;
+  } else {
+    reinforce_row_terms(expf(za[r] - row_max[r]) / row_sum[r], r, beta_logp, ret, method, K, L, g);
+  }
+  row_loss[r] = L;
+  row_g[r] = g;
 }
 
 // out[0] = sum of v[0..n) in a fixed order (one CTA)
@@ -248,12 +314,35 @@ static int64_t reinforce_partial_floats(const recnn_discrete_dims& d, int64_t ro
   return best;
 }
 
+// Split-K partial space of the item-streamed policy gradient: dW1, and dW2 of one chunk of every width up to `chunk`
+// (the last chunk may be narrower, and the split count depends on the width).  The split count is constant over
+// each run of 128 widths, so the widest of each run bounds it.  Independent of num_items.
+static int64_t streamed_partial_floats(const recnn_discrete_dims& d, int64_t rows, int chunk) {
+  int64_t best = 0;
+  for (int64_t top = 128;; top += 128) {
+    const int cw = (int)(top < chunk ? top : chunk);
+    for (int tcp = 0; tcp < 2; ++tcp) {
+      const int64_t f = (int64_t)dw_splits(cw, d.hidden, rows, tcp != 0) * cw * (d.hidden + 1);
+      if (f > best) best = f;
+    }
+    if (top >= chunk) break;
+  }
+  for (int tcp = 0; tcp < 2; ++tcp) {
+    const int64_t f = (int64_t)dw_splits(d.hidden, d.state_dim, rows, tcp != 0) * d.hidden * (d.state_dim + 1);
+    if (f > best) best = f;
+  }
+  return best;
+}
+
 struct DiscreteScratch {
   float *img, *h, *z, *dh, *row_loss, *partial;
+  float *row_max, *row_sum, *za, *row_g;     // item-streamed gradient only
   int* flags;
   int64_t floats;
 };
-static DiscreteScratch discrete_carve(const recnn_discrete_dims& d, int64_t n, bool backward, float* base) {
+// item_chunk > 0 (backward only): the item-streamed gradient, z holds one chunk of logits [n, item_chunk]
+static DiscreteScratch discrete_carve(const recnn_discrete_dims& d, int64_t n, bool backward, float* base,
+                                      int item_chunk = 0) {
   DiscreteScratch s;
   int64_t off = 0;
   auto take = [&](int64_t floats) {
@@ -265,11 +354,21 @@ static DiscreteScratch discrete_carve(const recnn_discrete_dims& d, int64_t n, b
   s.h = take(n * d.hidden);
   s.flags = reinterpret_cast<int*>(take(4));
   s.z = s.dh = s.row_loss = s.partial = nullptr;
+  s.row_max = s.row_sum = s.za = s.row_g = nullptr;
   if (backward) {
-    s.z = take(n * (int64_t)d.num_items);
+    const int chunk = item_chunk > 0 && item_chunk < d.num_items ? item_chunk : d.num_items;
+    s.z = take(n * (int64_t)chunk);
     s.dh = take(n * d.hidden);
     s.row_loss = take(n);
-    s.partial = take(reinforce_partial_floats(d, n));
+    if (item_chunk > 0) {
+      s.row_max = take(n);
+      s.row_sum = take(n);
+      s.za = take(n);
+      s.row_g = take(n);
+      s.partial = take(streamed_partial_floats(d, n, chunk));
+    } else {
+      s.partial = take(reinforce_partial_floats(d, n));
+    }
   }
   s.floats = off + 64;
   return s;
@@ -278,11 +377,10 @@ static float* align_floats(float* p) {      // 256-byte aligned start inside the
   return reinterpret_cast<float*>(round_up(reinterpret_cast<int64_t>(p), 256));
 }
 
-// logits = W2 relu(W1 s + b1) + b2 into z (row pitch num_items); h kept for the backward
-static int discrete_logits(const recnn_discrete_dims& d, const float* params, const float* state, int64_t n,
-                           const DiscreteScratch& s, float* z, cudaStream_t st, Seg* xs_out) {
+// h = relu(W1 s + b1) into s.h, kept for the backward
+static int discrete_hidden(const recnn_discrete_dims& d, const float* params, const float* state, int64_t n,
+                           const DiscreteScratch& s, cudaStream_t st, Seg* xs_out) {
   const DiscreteLayout l = discrete_layout(d);
-  const int H = d.hidden;
   recnn_dims dd;
   memset(&dd, 0, sizeof(dd));
   dd.state_dim = d.state_dim; dd.hidden = d.hidden; dd.action_dim = d.num_items;
@@ -290,9 +388,29 @@ static int discrete_logits(const recnn_discrete_dims& d, const float* params, co
   RECNN_PROPAGATE(repitch_state(dd, state, n, s.img, &xs, st));
   if (xs_out) *xs_out = xs;
   Rng rng = {nullptr, 0, nullptr};
-  RECNN_PROPAGATE(hidden_layer(xs, kNoSeg, params + l.w1, l.ld1, params + l.b1, H, n, false, nullptr, rng, 0, s.h, st));
+  return hidden_layer(xs, kNoSeg, params + l.w1, l.ld1, params + l.b1, d.hidden, n, false, nullptr, rng, 0, s.h, st);
+}
+
+// logits = W2 relu(W1 s + b1) + b2 into z (row pitch num_items); h kept for the backward
+static int discrete_logits(const recnn_discrete_dims& d, const float* params, const float* state, int64_t n,
+                           const DiscreteScratch& s, float* z, cudaStream_t st, Seg* xs_out) {
+  const DiscreteLayout l = discrete_layout(d);
+  const int H = d.hidden;
+  RECNN_PROPAGATE(discrete_hidden(d, params, state, n, s, st, xs_out));
   const Seg sh = {s.h, H, H, 0};
   return linear_out(sh, params + l.w2, l.ld2, params + l.b2, d.num_items, n, 0, nullptr, z, d.num_items, st);
+}
+
+// The logit GEMM of items [c0, c0 + cw) into s.z [n, cw] with epilogue EPI: EPI_LINEAR (the logits, as linear_out) or
+// EPI_DLOGITS (d loss / d logits).  Both passes of the streamed gradient run this one GEMM on the same operands without
+// split-K, so the logits the backward recomputes are bit-identical to those the statistics were taken from.
+template <int EPI>
+static int item_chunk_gemm(const recnn_discrete_dims& d, const float* params, const DiscreteScratch& s, int64_t n,
+                           int64_t c0, int cw, Epilogue e, cudaStream_t st) {
+  const DiscreteLayout l = discrete_layout(d);
+  const Seg sh = {s.h, d.hidden, d.hidden, 0};
+  e.out = s.z; e.ldo = cw; e.bias = params + l.b2 + c0;
+  return gemm_nt<EPI>(sh, kNoSeg, params + l.w2 + c0 * l.ld2, l.ld2, cw, n, e, st);
 }
 
 }  // namespace recnn
@@ -352,10 +470,9 @@ extern "C" int recnn_categorical_log_prob(const float* probs, int64_t n_rows, in
 }
 
 // out[0] = policy loss, out[1] = 1.0 if an action id was outside [0, num_items) (that row contributes nothing)
-extern "C" int recnn_reinforce_policy_grad(const recnn_discrete_dims* d, const float* params, float* grads,
-                                           const float* state, const int64_t* action, const float* beta_log_prob,
-                                           const float* returns, int64_t n_rows, int32_t method, int32_t top_k,
-                                           float* out, float* scratch, void* stream) {
+static int reinforce_args_ok(const recnn_discrete_dims* d, const float* params, float* grads, const float* state,
+                             const int64_t* action, const float* beta_log_prob, const float* returns, int64_t n_rows,
+                             int32_t method, int32_t top_k, float* out, float* scratch) {
   RECNN_REQUIRE(discrete_dims_ok(d) && params && grads && state && action && returns && out && scratch,
                 "null pointer / dims");
   RECNN_REQUIRE(method == RECNN_REINFORCE_BASIC || method == RECNN_REINFORCE_CORRECTED || method == RECNN_REINFORCE_TOPK,
@@ -363,6 +480,15 @@ extern "C" int recnn_reinforce_policy_grad(const recnn_discrete_dims* d, const f
   RECNN_REQUIRE(method == RECNN_REINFORCE_BASIC || beta_log_prob, "the corrected losses need the behaviour policy's log-probs");
   RECNN_REQUIRE(method != RECNN_REINFORCE_TOPK || top_k >= 1, "K >= 1");
   RECNN_REQUIRE(n_rows > 0, "no saved rows: select_action was never called since the last update");
+  return RECNN_OK;
+}
+
+extern "C" int recnn_reinforce_policy_grad(const recnn_discrete_dims* d, const float* params, float* grads,
+                                           const float* state, const int64_t* action, const float* beta_log_prob,
+                                           const float* returns, int64_t n_rows, int32_t method, int32_t top_k,
+                                           float* out, float* scratch, void* stream) {
+  RECNN_PROPAGATE(reinforce_args_ok(d, params, grads, state, action, beta_log_prob, returns, n_rows, method, top_k, out,
+                                    scratch));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const DiscreteLayout l = discrete_layout(*d);
   const int H = d->hidden, S = d->state_dim, I = d->num_items;
@@ -383,6 +509,66 @@ extern "C" int recnn_reinforce_policy_grad(const recnn_discrete_dims* d, const f
   RECNN_PROPAGATE(backprop_hidden(s.z, I, params + l.w2, l.ld2, H, 0, H, n_rows, s.h, 1.f, s.dh, st));
   RECNN_PROPAGATE(weight_grad(s.dh, H, xs, kNoSeg, n_rows, grads + l.w1, l.ld1, grads + l.b1, s.partial, st));
   (void)S;
+  RECNN_CHECK_CUDA(cudaMemcpyAsync(out + 1, s.flags, sizeof(int), cudaMemcpyDeviceToDevice, st));
+  return RECNN_OK;
+}
+
+extern "C" int64_t recnn_reinforce_streamed_scratch_floats(const recnn_discrete_dims* d, int64_t n_rows,
+                                                           int32_t item_chunk) {
+  if (!discrete_dims_ok(d) || n_rows <= 0 || item_chunk < 1) return 0;
+  return discrete_carve(*d, n_rows, true, nullptr, item_chunk).floats;
+}
+
+// recnn_reinforce_policy_grad without the [n_rows, num_items] logits: two passes over the item chunks [c0, c0 + C),
+// each recomputing the chunk's logits with the same GEMM.  Pass 1 takes each row's softmax statistics and the logit of
+// its action; pass 2 writes d logits straight from the GEMM epilogue and consumes them chunk by chunk.
+extern "C" int recnn_reinforce_policy_grad_streamed(const recnn_discrete_dims* d, const float* params, float* grads,
+                                                    const float* state, const int64_t* action,
+                                                    const float* beta_log_prob, const float* returns, int64_t n_rows,
+                                                    int32_t method, int32_t top_k, int32_t item_chunk, float* out,
+                                                    float* scratch, void* stream) {
+  RECNN_PROPAGATE(reinforce_args_ok(d, params, grads, state, action, beta_log_prob, returns, n_rows, method, top_k, out,
+                                    scratch));
+  RECNN_REQUIRE(item_chunk >= 1, "item_chunk >= 1");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const DiscreteLayout l = discrete_layout(*d);
+  const int H = d->hidden, I = d->num_items;
+  const int C = item_chunk < I ? item_chunk : I;
+  const long long* act = reinterpret_cast<const long long*>(action);
+  const DiscreteScratch s = discrete_carve(*d, n_rows, true, align_floats(scratch), item_chunk);
+  RECNN_CHECK_CUDA(cudaMemsetAsync(s.flags, 0, 4 * sizeof(int), st));
+  Seg xs;
+  RECNN_PROPAGATE(discrete_hidden(*d, params, state, n_rows, s, st, &xs));
+  // pass 1: per-row max, sum of exp and the action's logit over all items
+  for (int64_t c0 = 0; c0 < I; c0 += C) {
+    const int cw = (int)(I - c0 < C ? I - c0 : C);
+    RECNN_PROPAGATE(item_chunk_gemm<EPI_LINEAR>(*d, params, s, n_rows, c0, cw, base_epi(), st));
+    reinforce_chunk_stats_kernel<<<row_grid(n_rows), kRowThreads, 0, st>>>(s.z, n_rows, cw, c0, c0 == 0, act, s.row_max,
+                                                                          s.row_sum, s.za);
+    RECNN_CHECK_LAUNCH("reinforce_chunk_stats_kernel");
+  }
+  reinforce_streamed_terms_kernel<<<(unsigned)ceil_div(n_rows, 256), 256, 0, st>>>(
+      n_rows, I, act, s.row_max, s.row_sum, s.za, beta_log_prob, returns, method, top_k, s.row_loss, s.row_g, s.flags);
+  RECNN_CHECK_LAUNCH("reinforce_streamed_terms_kernel");
+  sum_rows_kernel<<<1, 1024, 0, st>>>(s.row_loss, n_rows, out);
+  RECNN_CHECK_LAUNCH("sum_rows_kernel");
+  // pass 2, per chunk: dz = d loss / d logits from the recomputed logits; dW2, db2 of the chunk's items;
+  // dh = sum over chunks of dz W2[chunk], gated by [h > 0] with the last chunk
+  const Seg sh = {s.h, H, H, 0};
+  Epilogue e = base_epi();
+  e.row_g = s.row_g; e.row_max = s.row_max; e.row_sum = s.row_sum; e.row_action = act;
+  for (int64_t c0 = 0; c0 < I; c0 += C) {
+    const int cw = (int)(I - c0 < C ? I - c0 : C);
+    const bool last = c0 + cw >= I;
+    e.col0 = c0;
+    RECNN_PROPAGATE(item_chunk_gemm<EPI_DLOGITS>(*d, params, s, n_rows, c0, cw, e, st));
+    RECNN_PROPAGATE(weight_grad(s.z, cw, sh, kNoSeg, n_rows, grads + l.w2 + c0 * l.ld2, l.ld2, grads + l.b2 + c0,
+                                s.partial, st));
+    RECNN_PROPAGATE(backprop_hidden(s.z, cw, params + l.w2 + c0 * l.ld2, l.ld2, H, 0, H, n_rows, last ? s.h : nullptr,
+                                    1.f, s.dh, st, c0 > 0));
+  }
+  // dW1 = dh^T s, db1 = colsum dh
+  RECNN_PROPAGATE(weight_grad(s.dh, H, xs, kNoSeg, n_rows, grads + l.w1, l.ld1, grads + l.b1, s.partial, st));
   RECNN_CHECK_CUDA(cudaMemcpyAsync(out + 1, s.flags, sizeof(int), cudaMemcpyDeviceToDevice, st));
   return RECNN_OK;
 }

@@ -250,8 +250,10 @@ static int linear_out(const Seg& x, const float* W, long long ldw, const float* 
 }
 
 // dX = (dZ W[:, col0:col0+K]) * gate(h)     dZ [n,C]; W [C, w_cols] row pitch ldw; out [n,K]
+// accumulate: dX = (out + dZ W[...]) * gate(h), i.e. one more term of a sum over blocks of C (gated by the last term)
 static int backprop_hidden(const float* dZ, int C, const float* W, long long ldw, int w_cols, int col0, int K,
-                           int64_t n, const float* h, float gate_scale, float* out, cudaStream_t st) {
+                           int64_t n, const float* h, float gate_scale, float* out, cudaStream_t st,
+                           bool accumulate = false) {
   Epilogue e = base_epi();
   e.out = out; e.ldo = K; e.h = h; e.ldh = K; e.gate_scale = gate_scale;
   const bool tc_ok = math_tc() && aligned16(dZ) && aligned16(W) && C % 4 == 0 && ldw % 4 == 0 && col0 % 4 == 0;
@@ -261,10 +263,12 @@ static int backprop_hidden(const float* dZ, int C, const float* W, long long ldw
     memset(&p, 0, sizeof(p));
     p.M = (int)n; p.N = K; p.K0 = C; p.b_k1_offset = C; p.b_n_offset = col0;
     const int bn = pick_bn(n, K);
-    const int r = h ? tc::launch<false, true, EPI_GATE>(a0, a1, b, p, 1, bn, e, st)
-                    : tc::launch<false, true, EPI_STORE>(a0, a1, b, p, 1, bn, e, st);
+    const int r = accumulate ? tc::launch<false, true, EPI_ACCUM>(a0, a1, b, p, 1, bn, e, st)
+                  : h ? tc::launch<false, true, EPI_GATE>(a0, a1, b, p, 1, bn, e, st)
+                      : tc::launch<false, true, EPI_STORE>(a0, a1, b, p, 1, bn, e, st);
     return r < 0 ? r : RECNN_OK;
   }
+  if (accumulate) return launch_gemm_simt<true, false, EPI_ACCUM>(mat(dZ, C), mat(W + col0, ldw), (int)n, K, C, 1, e, st);
   if (h) return launch_gemm_simt<true, false, EPI_GATE>(mat(dZ, C), mat(W + col0, ldw), (int)n, K, C, 1, e, st);
   return launch_gemm_simt<true, false, EPI_STORE>(mat(dZ, C), mat(W + col0, ldw), (int)n, K, C, 1, e, st);
 }

@@ -139,6 +139,8 @@ RECNN_TC_INST(true, true, EPI_STORE)
 RECNN_TC_INST(true, true, EPI_PARTIAL)
 RECNN_TC_INST(false, false, EPI_PARTIAL)
 RECNN_TC_INST(true, false, EPI_STORE)
+RECNN_TC_INST(false, false, EPI_DLOGITS)
+RECNN_TC_INST(false, true, EPI_ACCUM)
 
 }  // namespace tc
 }  // namespace recnn

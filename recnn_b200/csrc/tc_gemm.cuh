@@ -313,6 +313,12 @@ __device__ __forceinline__ void epilogue_row(const Epilogue& e, const Problem& p
   float* out_row;
   if (EPI == EPI_PARTIAL) out_row = e.out + ((long long)z * p.M + m) * e.ldo + p.n_out_offset;
   else out_row = e.out + (long long)m * e.ldo + p.n_out_offset;
+  float row_g = 0.f, row_max = 0.f, row_sum = 1.f;
+  long long row_item = 0;                  // EPI_DLOGITS: the drawn action as a column of this output
+  if (EPI == EPI_DLOGITS) {
+    row_g = e.row_g[m]; row_max = e.row_max[m]; row_sum = e.row_sum[m];
+    row_item = e.row_action[m] - e.col0;
+  }
 #pragma unroll
   for (int j0 = 0; j0 < NC; j0 += W) {
     if (nb + j0 < N) {
@@ -371,6 +377,11 @@ __device__ __forceinline__ void epilogue_row(const Epilogue& e, const Problem& p
                 }
               } else if (EPI == EPI_GATE) {
                 x = e.h[(long long)m * e.ldh + nn] > 0.f ? x * e.gate_scale : 0.f;
+              } else if (EPI == EPI_DLOGITS) {
+                x = dlogit(row_g, x + __ldg(e.bias + nn), row_max, row_sum, nn == row_item);
+              } else if (EPI == EPI_ACCUM) {
+                x = out_row[nn] + x;
+                if (e.h) x = e.h[(long long)m * e.ldh + nn] > 0.f ? x * e.gate_scale : 0.f;
               }
             }
             v[u] = x;

@@ -1,7 +1,8 @@
 """Drop-in for recnn.nn.update.reinforce (recnn/nn/update/reinforce.py:10-129): ChooseREINFORCE and reinforce_update.
 
 The policy loss and its gradient are ONE device call (recnn_reinforce_policy_grad: recomputed forward, closed-form
-d loss / d logits, three tensor-core GEMMs) over the rows ``DiscreteActor`` saved since the last policy update; the
+d loss / d logits, three tensor-core GEMMs; past 1 GiB of logits its item-streamed form, which never holds more than one
+chunk of them) over the rows ``DiscreteActor`` saved since the last policy update; the
 optimizer step is the fused arena kernel (recnn_b200.optim) or any torch optimizer stepping the aliased ``.grad``
 views.  The critic half is the DDPG critic step (value_update) fed with the target policy's probabilities.
 """
@@ -16,6 +17,19 @@ from ... import utils
 from ...utils.misc import DummyWriter
 from ..arena import param_arena, grad_arena
 from .misc import value_update
+
+
+_MAX_LOGIT_FLOATS = 1 << 28          # 1 GiB of fp32 logits
+
+
+def _policy_grad_plan(rows, items):
+    """Item chunk width of the policy gradient over ``rows`` saved rows and ``items`` outputs; 0 = materialise.
+
+    Up to 1 GiB of logits the materialised entry (one logits GEMM, 3/4 of the streamed FLOPs) is used; beyond, the
+    item-streamed entry with the widest multiple of 128 whose [rows, chunk] logits stay within 1 GiB (at least 128)."""
+    if rows * items <= _MAX_LOGIT_FLOATS:
+        return 0
+    return max(128, _MAX_LOGIT_FLOATS // rows // 128 * 128)
 
 
 def _policy_loss(policy, returns, method):
@@ -44,16 +58,22 @@ def _policy_loss(policy, returns, method):
     n = state.shape[0]
     d = policy.dims
     L = _lib.lib()
-    scratch = torch.empty(L.recnn_discrete_scratch_floats(d, n, 1), device=dev, dtype=torch.float32)
+    chunk = _policy_grad_plan(n, d.num_items)
+    floats = L.recnn_reinforce_streamed_scratch_floats(d, n, chunk) if chunk else L.recnn_discrete_scratch_floats(d, n, 1)
+    scratch = torch.empty(floats, device=dev, dtype=torch.float32)
     out = torch.zeros(2, device=dev, dtype=torch.float32)
     ks = {r.get("K") for r in saved if r.get("K") is not None}
     if len(ks) > 1:
         raise ValueError("select_action was called with different K since the last policy update: %s" % sorted(ks))
     K = ks.pop() if ks else 1
+    args = (d, flat.data_ptr(), grads.data_ptr(), state.data_ptr(), action.data_ptr(), _lib.ptr(beta_lp),
+            ret_rows.data_ptr(), n, method, K)
     with torch.cuda.device(dev):
-        _lib.check(L.recnn_reinforce_policy_grad(d, flat.data_ptr(), grads.data_ptr(), state.data_ptr(), action.data_ptr(),
-                                                 _lib.ptr(beta_lp), ret_rows.data_ptr(), n, method, K, out.data_ptr(),
-                                                 scratch.data_ptr(), _lib.stream_ptr(dev)))
+        if chunk:
+            _lib.check(L.recnn_reinforce_policy_grad_streamed(*args, chunk, out.data_ptr(), scratch.data_ptr(),
+                                                              _lib.stream_ptr(dev)))
+        else:
+            _lib.check(L.recnn_reinforce_policy_grad(*args, out.data_ptr(), scratch.data_ptr(), _lib.stream_ptr(dev)))
     if int(out.view(torch.int32)[1].item()) != 0:
         raise IndexError("saved action index out of range for the policy's output layer")
     return out[0].clone()

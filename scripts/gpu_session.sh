@@ -28,6 +28,9 @@ except Exception as e:
     print("bench failed:", e); print(open("$O/${tag}_bench.err").read()[-2000:])
 PY
 
+el "3. REINFORCE policy gradient against the vocabulary size"
+timeout 900 python scripts/bench_reinforce_vocab.py > $O/${tag}_reinforce_vocab.jsonl 2> $O/${tag}_reinforce_vocab.err
+
 if [ "$2" != "skip-ncu" ]; then
 el "4. ncu: launch list of the step"
 timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -c 900 --csv --log-file $O/${tag}_launches.csv \
