@@ -98,7 +98,5 @@ def enable_data_parallel(agent_or_nets, group=None, sync_weights=True):
             warnings.warn("recnn_b200: %s; falling back to NCCL all-reduces between the step's phases" % exc)
     policy.__dict__["_recnn_dp"] = (group, world, comm)
     for eng in policy.__dict__.get("_recnn_engines", {}).values():
-        eng.group, eng.world, eng.comm = group, world, comm
-        eng.graphs.clear()
-        eng._fast.clear()
+        eng.set_data_parallel(group, world, comm)
     return agent_or_nets

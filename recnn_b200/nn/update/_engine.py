@@ -4,8 +4,8 @@ Responsibilities (all plumbing; the arithmetic is in recnn_b200/csrc):
   * validate / (re)build the flat parameter, gradient and optimizer arenas;
   * stage the batch into fixed device buffers (one async copy per tensor) so the
     step is replayable as a CUDA graph;
-  * pick the phase split: one call (built-in optimizers, one GPU), or three
-    calls with gradient all-reduces / external ``optimizer.step()`` in between;
+  * run the phase schedule of the update (``schedule``): which phase masks go to the C
+    side, and which all-reduces / external ``optimizer.step()`` calls run between them;
   * read the 3-4 loss scalars back (the only synchronisation of a step -- the
     reference API returns Python floats, recnn/nn/update/ddpg.py:102).
 """
@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import os
 import warnings
+from typing import NamedTuple
 
 import torch
 
@@ -21,12 +22,79 @@ from ... import optim as _optim
 from ..arena import param_arena, grad_arena
 
 _USE_GRAPHS = os.environ.get("RECNN_B200_GRAPHS", "1") != "0"
+_MAX_GRAPH_KEYS = 16            # bound of the graph cache (first sightings included)
 MASK_KEY = "dropout_masks"      # optional batch entries for bit-reproducible runs
 NOISE_KEY = "noise"
 
 DDPG_NETS = ("value_net", "target_value_net", "policy_net", "target_policy_net")
 TD3_NETS = ("value_net1", "target_value_net1", "value_net2", "target_value_net2", "policy_net",
             "target_policy_net")
+
+# Host actions that run between two C calls of a step, on the step's stream.
+ALLREDUCE_VALUE_GRADS = "allreduce_value_grads"
+ALLREDUCE_POLICY_GRADS = "allreduce_policy_grads"
+ALLREDUCE_LOSSES = "allreduce_losses"
+STEP_VALUE_OPTIMIZERS = "step_value_optimizers"
+STEP_POLICY_OPTIMIZER = "step_policy_optimizer"
+
+
+class Schedule(NamedTuple):
+    segments: tuple     # ((phase mask, (host action, ...)), ...): C calls in order, each followed by its host actions
+    capturable: bool    # may run as one CUDA graph per segment (the host actions stay between the replays)
+
+
+def schedule(value_only, learn, do_policy, value_builtin, policy_builtin, debug, world, peer_comm) -> Schedule:
+    """The C calls of one update and the host work between them (the same for DDPG and TD3: the host actions
+    on the value gradients / optimizers cover both of TD3's critics).
+
+    A learning step whose optimizers are all built in runs fused: one call with every phase, its gradient
+    exchange inside the kernels when there is one GPU or a peer communicator; with NCCL it is cut into three
+    calls where the critic and then the actor gradients are complete.  Only these fused steps are captured
+    into CUDA graphs.  Anything else -- an external optimizer, learn=False (debug outputs), the critic-only
+    ``value_only`` step -- runs phase by phase with direct launches: a built-in optimizer is the C side's
+    optimizer phase, an external one is stepped in Python, and with several ranks the gradients and the loss
+    scalars go through NCCL between the calls."""
+    P = _lib
+    if learn and not value_only and not debug and value_builtin and policy_builtin:
+        if world == 1 or peer_comm:
+            return Schedule(((P.PH_ALL, ()),), True)
+        grads = (ALLREDUCE_POLICY_GRADS,) if do_policy else ()
+        return Schedule(((P.PH_GATHER | P.PH_VALUE_GRAD, (ALLREDUCE_VALUE_GRADS,)),
+                         (P.PH_VALUE_OPT | P.PH_POLICY_LOSS | P.PH_POLICY_GRAD, grads + (ALLREDUCE_LOSSES,)),
+                         (P.PH_POLICY_OPT | P.PH_SOFT_UPDATE | P.PH_FINISH, ())), True)
+    dp = world > 1
+    segs = []
+
+    def call(phases):
+        segs.append((phases, []))
+
+    def then(action):
+        segs[-1][1].append(action)
+
+    call(P.PH_GATHER | P.PH_VALUE_GRAD)
+    if learn:
+        if dp:
+            then(ALLREDUCE_VALUE_GRADS)
+        if value_builtin:
+            call(P.PH_VALUE_OPT)
+        else:
+            then(STEP_VALUE_OPTIMIZERS)
+    if not value_only:
+        call(P.PH_POLICY_LOSS)
+        if do_policy:
+            call(P.PH_POLICY_GRAD)
+            if dp:
+                then(ALLREDUCE_POLICY_GRADS)
+            # clip coefficient (+ the fused optimizer when the policy optimizer is built in; for an
+            # external one the C side only scales the gradient in place)
+            call(P.PH_POLICY_OPT)
+            if not policy_builtin:
+                then(STEP_POLICY_OPTIMIZER)
+            call(P.PH_SOFT_UPDATE)
+    if dp:
+        then(ALLREDUCE_LOSSES)
+    call(P.PH_FINISH)                    # ++rng_step, losses -> pinned host
+    return Schedule(tuple((ph, tuple(acts)) for ph, acts in segs), False)
 
 
 class StepEngine:
@@ -59,11 +127,8 @@ class StepEngine:
             raise ValueError("critic shape does not match the actor (expects input state_dim+action_dim, same hidden, 1 output)")
         self.n_rows = -1
         self.form = None
-        self.graphs = {}
-        self.seg_graphs = {}
-        self._fast = {}
-        self.graph_sig = None
-        self.eager_runs = {}
+        self.graphs = {}             # bytes(StepArgs) -> None once run directly, then [(CUDAGraph, kernels)] per segment
+        self._fast = {}              # (value_only, do_policy, form, n) -> (tokens, StepArgs, Schedule, graphs)
         self.group = None            # torch.distributed process group for data parallel
         self.world = 1
         self.comm = None             # recnn_b200.dist.PeerComm: in-kernel all-reduce over NVLink peer memory
@@ -77,18 +142,21 @@ class StepEngine:
         self._probes = {}            # net name -> (module, first parameter, last parameter): see _tokens
         self._params_seen, self._params_version = None, 0
         self.kernels = 0             # kernels of this library launched by this engine (graph replays included)
-        self.last_call_kernels = 0
+
+    def set_data_parallel(self, group, world, comm):
+        """Exchange gradients and losses over ``group`` (``world`` ranks), in the step's kernels through the
+        peer communicator ``comm`` or, when it is None, with NCCL between the step's phases."""
+        self.group, self.world, self.comm = group, world, comm
+        self._invalidate()
 
     # ------------------------------------------------------------------ staging
     def _invalidate(self):
-        """Drop everything that baked device addresses in: captured graphs (whole-step and per-segment),
-        the fast-path table of (tokens -> graph / cached StepArgs) and the first-sight bookkeeping.  Called
-        whenever a staging buffer or the workspace is (re)allocated, the batch shape changes, or data
-        parallelism is (re)configured -- a stale graph would run against freed memory."""
+        """Drop everything that baked device addresses or the schedule in: the graph cache (first sightings
+        included) and the fast-path table.  Called whenever a staging buffer or the workspace is (re)allocated,
+        the batch shape changes, or data parallelism is (re)configured -- a stale graph would run against freed
+        memory."""
         self.graphs.clear()
-        self.seg_graphs.clear()
         self._fast.clear()
-        self.eager_runs.clear()
 
     def _buffer(self, name, shape, dtype):
         b = self.buf.get(name)
@@ -266,124 +334,80 @@ class StepEngine:
         a.workspace_bytes = ws.numel()
         return a, pol_opt, val_opts
 
-    def _signature(self, a):
-        """Everything a captured graph baked in: pointers and scalars."""
-        return bytes(a)
-
-    def _launch(self, a, phases, want_debug=None):
+    def _launch(self, a, phases):
+        """One C call of the step on the current stream; returns the number of kernels it launched."""
         a.phases = phases
-        if want_debug is not None:
-            a.next_action_out = _lib.ptr(want_debug.get("next_action"))
-            a.gen_action_out = _lib.ptr(want_debug.get("gen_action"))
         L = _lib.lib()
         fn = L.recnn_ddpg_step if self.algo == _lib.ALGO_DDPG else L.recnn_td3_step
         before = L.recnn_b200_launch_count()
         _lib.check(fn(a, _lib.stream_ptr(self.device)))
-        self.last_call_kernels = L.recnn_b200_launch_count() - before
-        self.kernels += self.last_call_kernels
+        return L.recnn_b200_launch_count() - before
 
-    def _body(self, a, nets, do_policy):
-        """The whole step with built-in optimizers: one C call on one GPU.  (The multi-GPU branch below
-        is kept for direct launches only: capturing the NCCL all-reduces into the step graph deadlocked
-        on the 2-GPU box, so data parallel runs go through the split-phase path in _step.)"""
-        P = _lib
-        if self.world == 1 or a.comm:      # with a peer communicator the gradient all-reduces are kernels of the step
-            self._launch(a, P.PH_ALL)
-            return self.last_call_kernels
-        td3 = self.algo == P.ALGO_TD3
-        kernels = 0
-        self._launch(a, P.PH_GATHER | P.PH_VALUE_GRAD)
-        kernels += self.last_call_kernels
-        for i in range(2 if td3 else 1):
-            self._allreduce(grad_arena(nets["value_net" + (str(i + 1) if td3 else "")]))
-        self._launch(a, P.PH_VALUE_OPT | P.PH_POLICY_LOSS | P.PH_POLICY_GRAD)
-        kernels += self.last_call_kernels
-        if do_policy:
+    def _allreduce(self, t):
+        import torch.distributed as dist
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
+
+    def _host_action(self, action, nets, pol_opt, val_opts):
+        value_nets = [nets[k] for k in self.names if k.startswith("value_net")]
+        if action == ALLREDUCE_VALUE_GRADS:
+            for vn in value_nets:
+                self._allreduce(grad_arena(vn))
+        elif action == ALLREDUCE_POLICY_GRADS:
             self._allreduce(grad_arena(nets["policy_net"]))
-        self._allreduce(self.losses[:3])
-        self._launch(a, P.PH_POLICY_OPT | P.PH_SOFT_UPDATE | P.PH_FINISH)
-        kernels += self.last_call_kernels
-        return kernels
+        elif action == ALLREDUCE_LOSSES:
+            self._allreduce(self.losses[:3])
+        elif action == STEP_VALUE_OPTIMIZERS:
+            for vn, vo in zip(value_nets, val_opts):
+                grad_arena(vn)          # re-attach p.grad views if zero_grad(set_to_none) dropped them
+                vo.step()
+        else:
+            assert action == STEP_POLICY_OPTIMIZER, action
+            grad_arena(nets["policy_net"])
+            pol_opt.step()
 
-    def _run_fused(self, a, nets, do_policy):
-        """Direct launches the first time a variant is seen, then one CUDA graph (kernels, side-stream
-        forks/joins, the loss read-back and -- with several GPUs -- the NCCL all-reduces) per variant."""
-        a.phases = _lib.PH_ALL
-        key = self._signature(a)
-        if not _USE_GRAPHS:
-            self._body(a, nets, do_policy)
-            return None
-        g = self.graphs.get(key)
-        if g is not None:
-            g[0].replay()
-            self.kernels += g[1]
-            return g
-        runs = self.eager_runs.get(key, 0)
-        if len(self.eager_runs) > 256:    # variable-size minibatches (reference-style FrameEnv batches): every step is
-            self.eager_runs.clear()       # a new variant; do not let the bookkeeping grow with the run
-        self.eager_runs[key] = runs + 1
-        if runs < 1:                      # first time: plain launch (also warms lazy module loading)
-            self._body(a, nets, do_policy)
-            return None
-        if len(self.graphs) > 16:
-            self._invalidate()
-        try:
-            torch.cuda.synchronize(self.device)
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                n_kernels = self._body(a, nets, do_policy)
-            self.graphs[key] = (g, n_kernels)
-            g.replay()
-            self.kernels += n_kernels
-            return self.graphs[key]
-        except Exception as exc:      # capture unsupported in this context: stay on direct launches
-            warnings.warn("recnn_b200: CUDA graph capture failed (%s); using direct launches" % exc)
-            globals()["_USE_GRAPHS"] = False
-            self._body(a, nets, do_policy)
-            return None
-
-    def _run_segments(self, a, nets, do_policy, vkey):
-        """Data parallel: the step is cut where gradients are complete.  Each cut piece is its own CUDA
-        graph (kernels only); the NCCL all-reduces run between the replays on the same stream."""
-        P = _lib
-        td3 = self.algo == P.ALGO_TD3
-        segs = (P.PH_GATHER | P.PH_VALUE_GRAD, P.PH_VALUE_OPT | P.PH_POLICY_LOSS | P.PH_POLICY_GRAD,
-                P.PH_POLICY_OPT | P.PH_SOFT_UPDATE | P.PH_FINISH)
+    def _graphs(self, a, sched):
+        """The CUDA graphs of a capturable schedule with these arguments: None the first time they are seen
+        (direct launches, which also warm lazy module loading) or when capture fails, captured the second time.
+        Keyed by the arguments' bytes, i.e. every pointer and scalar the graphs bake in."""
         a.phases = 0
-        key = self._signature(a)
-        ent = self.seg_graphs.get(key)
-        runs = self.eager_runs.get(key, 0)
-        self.eager_runs[key] = runs + 1
-        if ent is None and _USE_GRAPHS and runs >= 1:
+        key = bytes(a)
+        if key not in self.graphs:
+            if len(self.graphs) >= _MAX_GRAPH_KEYS:     # e.g. hyper-parameters that change every step
+                self._invalidate()
+            self.graphs[key] = None
+            return None
+        graphs = self.graphs[key]
+        if graphs is None:
             try:
                 torch.cuda.synchronize(self.device)
-                ent = []
-                for ph in segs:
+                graphs = []
+                for phases, _ in sched.segments:
                     g = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(g):
-                        self._launch(a, ph)
-                    ent.append((g, self.last_call_kernels))
-                self.seg_graphs[key] = ent
-            except Exception as exc:
+                        n = self._launch(a, phases)
+                    graphs.append((g, n))
+            except Exception as exc:      # capture unsupported in this context: stay on direct launches
                 warnings.warn("recnn_b200: CUDA graph capture failed (%s); using direct launches" % exc)
                 globals()["_USE_GRAPHS"] = False
-                ent = None
+                return None
+            self.graphs[key] = graphs
+        return graphs
 
-        def run(i):
-            if ent is not None:
-                ent[i][0].replay()
-                self.kernels += ent[i][1]
+    def _run(self, a, sched, nets, pol_opt=None, val_opts=None, graphs=None):
+        """Every segment of the schedule -- a graph replay or a direct C call -- followed by its host actions.
+        Returns the graphs used (None: direct launches)."""
+        if graphs is None and sched.capturable and _USE_GRAPHS:
+            graphs = self._graphs(a, sched)
+        for i, (phases, actions) in enumerate(sched.segments):
+            if graphs is not None:
+                g, n = graphs[i]
+                g.replay()
             else:
-                self._launch(a, segs[i])
-
-        run(0)
-        for i in range(2 if td3 else 1):
-            self._allreduce(grad_arena(nets["value_net" + (str(i + 1) if td3 else "")]))
-        run(1)
-        if do_policy:
-            self._allreduce(grad_arena(nets["policy_net"]))
-        self._allreduce(self.losses[:3])
-        run(2)
+                n = self._launch(a, phases)
+            self.kernels += n
+            for act in actions:
+                self._host_action(act, nets, pol_opt, val_opts)
+        return graphs
 
     def _read_losses(self):
         """After the stream synchronisation of a step: the loss scalars, or the step's error."""
@@ -395,15 +419,6 @@ class StepEngine:
             raise _lib.RecnnError("data parallel: the ranks disagree on the global row count; pass "
                                   "batch['n_rows_global'] when the shards are uneven")
         return self.losses_host[:4].tolist()
-
-    # ------------------------------------------------------------------ the step
-    def step(self, batch, params, nets, optimizer, learn, step, debug, policy_every_key):
-        with torch.cuda.device(self.device):
-            return self._step(batch, params, nets, optimizer, learn, step, debug, policy_every_key)
-
-    def _allreduce(self, t):
-        import torch.distributed as dist
-        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
 
     def _tokens(self, nets, optimizer, params, st):
         """Cheap fingerprint of everything a cached StepArgs / CUDA graph depends on: storage addresses of the nets
@@ -444,115 +459,52 @@ class StepEngine:
                     0 if self.comm is None else self.comm.ptr))
         return tok
 
-    def _step(self, batch, params, nets, optimizer, learn, step, debug, policy_every_key):
-        st = self._stage_batch(batch)
+    # ------------------------------------------------------------------ the step
+    def step(self, batch, params, nets, optimizer, learn, step, debug, policy_every_key):
+        """One DDPG / TD3 update (recnn/nn/update/ddpg.py, td3.py)."""
         do_policy = bool(learn and step % params[policy_every_key] == 0)
-        td3 = self.algo == _lib.ALGO_TD3
-        # ---- fast path: same variant as a previous step -> replay its graph
-        if learn and _USE_GRAPHS:
-            vkey = (do_policy, st["form"], st["n"])
-            ent = self._fast.get(vkey)
-            tok = self._tokens(nets, optimizer, params, st)
-            if ent is not None and ent[0] == tok:
-                if self.world == 1 or self.comm is not None:
-                    ent[1].replay()
-                    self.kernels += ent[2]
-                else:
-                    self._run_segments(ent[1], nets, do_policy, None)      # cached StepArgs
-                torch.cuda.current_stream(self.device).synchronize()
-                return self._read_losses()
+        with torch.cuda.device(self.device):
+            return self._update(batch, params, nets, optimizer, learn, do_policy, debug, False)
+
+    def value_only(self, batch, params, nets, optimizer, learn, debug):
+        """recnn/nn/update/misc.py:10-55 on its own: critic step without the policy half."""
+        with torch.cuda.device(self.device):
+            return self._update(batch, params, nets, optimizer, learn, False, debug, True)
+
+    def _update(self, batch, params, nets, optimizer, learn, do_policy, debug, value_only):
+        st = self._stage_batch(batch)
+        if value_only and self.discrete:
+            # next_action = target_policy_net(next_state)   (misc.py:28 with a DiscreteActor: probabilities)
+            st["next_action"] = self._stage("next_action", nets["target_policy_net"](st["next_state"]), torch.float32)
+        # ---- fast path: same variant as a previous step -> replay its graphs
+        vkey = (value_only, do_policy, st["form"], st["n"])
+        ent = self._fast.get(vkey) if learn and _USE_GRAPHS else None
+        if ent is not None and ent[0] == self._tokens(nets, optimizer, params, st):
+            self._run(ent[1], ent[2], nets, graphs=ent[3])
+            torch.cuda.current_stream(self.device).synchronize()
+            return self._read_losses()
         a, pol_opt, val_opts = self._build_args(st, nets, optimizer, params, learn, do_policy)
-        builtin = (not learn) or (isinstance(pol_opt, _optim._ArenaOptimizer)
-                                  and all(isinstance(v, _optim._ArenaOptimizer) for v in val_opts))
         want_debug = None
         if not learn:
             n, A = st["n"], self.dims.action_dim
-            want_debug = {"next_action": torch.empty(n, A, device=self.device),
-                          "gen_action": torch.empty(n, A, device=self.device)}
-        fused = builtin and learn and want_debug is None
-        if fused and self.comm is not None:
-            a.comm = self.comm.ptr
-        if fused and self.world > 1 and self.comm is None:
-            self._run_segments(a, nets, do_policy, None)
-            if _USE_GRAPHS:
-                self._fast[(do_policy, st["form"], st["n"])] = (self._tokens(nets, optimizer, params, st), a, 0)
-            torch.cuda.current_stream(self.device).synchronize()
-            return self._read_losses()
-        if fused:
-            g = self._run_fused(a, nets, do_policy)
-            if g is not None:
-                # arenas may have been (re)built by _build_args: fingerprint after the fact
-                self._fast[(do_policy, st["form"], st["n"])] = (self._tokens(nets, optimizer, params, st), g[0], g[1])
-            torch.cuda.current_stream(self.device).synchronize()
-            return self._read_losses()
-        else:
-            P = _lib
-            value_nets = [nets["value_net" + (str(i + 1) if td3 else "")] for i in range(2 if td3 else 1)]
-            self._launch(a, P.PH_GATHER | P.PH_VALUE_GRAD, want_debug)
-            if learn:
-                if self.world > 1:
-                    for vn in value_nets:
-                        self._allreduce(grad_arena(vn))
-                # Each optimizer is stepped exactly once, by whoever owns it: the C side runs the fused
-                # SGD/Adam of a built-in optimizer (a.value_optim.kind != EXTERNAL), Python steps anything else.
-                if a.value_optim.kind != P.OPT_EXTERNAL:
-                    self._launch(a, P.PH_VALUE_OPT, want_debug)
-                else:
-                    for vn, vo in zip(value_nets, val_opts):
-                        grad_arena(vn)          # re-attach p.grad views if zero_grad(set_to_none) dropped them
-                        vo.step()
-            self._launch(a, P.PH_POLICY_LOSS, want_debug)
-            if do_policy:
-                self._launch(a, P.PH_POLICY_GRAD, want_debug)
-                if self.world > 1:
-                    self._allreduce(grad_arena(nets["policy_net"]))
-                # clip coefficient (+ the fused optimizer when the policy optimizer is built in; for an
-                # external one the C side only scales the gradient in place)
-                self._launch(a, P.PH_POLICY_OPT, want_debug)
-                if a.policy_optim.kind == P.OPT_EXTERNAL:
-                    grad_arena(nets["policy_net"])
-                    pol_opt.step()
-                self._launch(a, P.PH_SOFT_UPDATE, want_debug)
-            if self.world > 1:
-                self._allreduce(self.losses[:3])
-            self._launch(a, P.PH_FINISH, want_debug)     # ++rng_step, losses -> pinned host
+            want_debug = {k: torch.empty(n, A, device=self.device)
+                          for k in (("next_action",) if value_only else ("next_action", "gen_action"))}
+            a.next_action_out = _lib.ptr(want_debug.get("next_action"))
+            a.gen_action_out = _lib.ptr(want_debug.get("gen_action"))
+        sched = schedule(value_only, learn, do_policy, isinstance(val_opts[0], _optim._ArenaOptimizer),
+                         isinstance(pol_opt, _optim._ArenaOptimizer), want_debug is not None, self.world,
+                         self.comm is not None)
+        if sched.capturable and self.comm is not None:
+            a.comm = self.comm.ptr        # the fused step all-reduces in its kernels
+        graphs = self._run(a, sched, nets, pol_opt, val_opts)
+        if graphs is not None:
+            # arenas may have been (re)built by _build_args: fingerprint after the fact
+            self._fast[vkey] = (self._tokens(nets, optimizer, params, st), a, sched, graphs)
         torch.cuda.current_stream(self.device).synchronize()
         vals = self._read_losses()
-        if want_debug is not None:
-            debug["next_action"] = want_debug["next_action"]
-            debug["gen_action"] = want_debug["gen_action"]
+        for k, t in (want_debug or {}).items():
+            debug[k] = t                  # debug=None fails like the reference (misc.py:47)
         return vals
-
-
-def _value_only(self, batch, params, nets, optimizer, learn, debug):
-    """recnn/nn/update/misc.py:10-55 on its own: critic step without the policy half."""
-    with torch.cuda.device(self.device):
-        st = self._stage_batch(batch)
-        if self.discrete:
-            # next_action = target_policy_net(next_state)   (misc.py:28 with a DiscreteActor: probabilities)
-            st["next_action"] = self._stage("next_action", nets["target_policy_net"](st["next_state"]), torch.float32)
-        a, _, val_opts = self._build_args(st, nets, optimizer, params, learn, False)
-        want_debug = None
-        if not learn:
-            want_debug = {"next_action": torch.empty(st["n"], self.dims.action_dim, device=self.device)}
-        self._launch(a, _lib.PH_GATHER | _lib.PH_VALUE_GRAD, want_debug)
-        if learn:
-            vn = nets["value_net"]
-            if self.world > 1:
-                self._allreduce(grad_arena(vn))
-            if isinstance(val_opts[0], _optim._ArenaOptimizer):
-                self._launch(a, _lib.PH_VALUE_OPT, want_debug)
-            else:
-                grad_arena(vn)
-                val_opts[0].step()
-        self._launch(a, _lib.PH_FINISH, want_debug)
-        torch.cuda.current_stream(self.device).synchronize()
-        if want_debug is not None:
-            debug["next_action"] = want_debug["next_action"]
-        return self._read_losses()
-
-
-StepEngine.value_only = _value_only
 
 
 def get_engine(algo, nets, device) -> StepEngine:
@@ -566,6 +518,6 @@ def get_engine(algo, nets, device) -> StepEngine:
         eng = StepEngine(algo, nets, dev)
         dp = policy.__dict__.get("_recnn_dp")
         if dp is not None:
-            eng.group, eng.world, eng.comm = dp
+            eng.set_data_parallel(*dp)
         cache[key] = eng
     return eng
